@@ -6,7 +6,7 @@ synthetic 16 kHz int16 audio: 65 536 streams x 3 s (= 300 ten-ms frames, 100 mod
 per GPU -- BASELINE.json configs[1].  Streams are independent, so N GPUs run N shards of 65 536
 streams each with no data-path collective (weak scaling; configs[4] = 8 x 65 536 = 524 288 streams).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--model f32|int8]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--model f32|int8] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Keys beyond the driver contract:
   roofline      dominant kernel (K1 spectral) achieved algorithmic GB/s vs MEASURED_PEAKS.json
@@ -19,6 +19,7 @@ One JSON line on stdout (rank 0).  Keys beyond the driver contract:
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -40,6 +41,7 @@ FRAMES_PER_STEP = SAMPLES_PER_STEP // 160
 K1_ALG_BYTES_PER_FRAME = 320      # 160 new int16 samples per 10 ms frame: the only mandatory HBM traffic of K1 (DESIGN.md)
 METRIC = "streams_x_frames_per_sec"
 UNIT = "frames/s"
+DUMP_BYTES = 64 * 10**6           # --dump-outputs: at most this much in all
 
 
 def parse_args():
@@ -63,7 +65,29 @@ def parse_args():
                     help="skip the legs for the other BASELINE.json configurations (the other model dtype in clip mode, live 30 ms steps "
                          "for both dtypes, feature extractor only)")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the probabilities the last timed step returned as DIR/probs.npy (float32); the "
+                         "input audio is seeded, so runs with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy in float32.  An array larger than its share of DUMP_BYTES keeps a fixed sample
+    of its rows (streams): np.random.default_rng(0).choice(rows, k, replace=False), in stream order, so every run with the
+    same arguments writes the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096            # room for the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // a[0].nbytes, replace=False))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def model_blob(kind: str) -> bytes:
@@ -211,16 +235,19 @@ class ClockSampler:
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
         except OSError:
             self.proc = None
+        atexit.register(self.stop)          # the sampler must not outlive a benchmark that fails before stop()
 
     def stop(self):
         out = {"sm_mhz": None, "sm_max_mhz": None, "reasons": []}
-        if self.proc is None:
+        proc, self.proc = self.proc, None
+        if proc is None:
             return out
-        self.proc.terminate()
+        proc.terminate()
         try:
-            self.proc.wait(timeout=5)
+            proc.wait(timeout=5)
         except subprocess.TimeoutExpired:
-            self.proc.kill()
+            proc.kill()
+            proc.wait()
         sm, mx, reasons = [], [], set()
         try:
             for ln in open(self.path):
@@ -354,10 +381,16 @@ def run_gpu(args):
     barrier()
     l0 = eng.launch_count
     eng.profile(True)
-    ms_resident = timed(lambda: eng.predict_clip(audio, out=probs), args.steps)
+    last = {}
+
+    def resident_step():
+        last["probs"] = eng.predict_clip(audio, out=probs)
+    ms_resident = timed(resident_step, args.steps)
     launches = (eng.launch_count - l0)
     prof = eng.profile_read()
     eng.profile(False)
+    # what the last timed step returned, copied before the legs below reuse `probs`
+    outputs = {"probs": last["probs"].cpu().numpy()} if args.dump_outputs and world == 1 else None
     checksum = float(probs[:, :100].double().sum().item())
     kernels = {k: {"ms_per_step": v[0] / args.steps, "launches_per_step": v[1] / args.steps} for k, v in prof.items()}
 
@@ -413,6 +446,8 @@ def run_gpu(args):
             ingest_step()
         l0 = count_launches()
         ms_per_step = timed(ingest_step, args.steps)
+        if args.dump_outputs and rank == 0:
+            outputs = {"probs": gathered.cpu().numpy()}
         lt = torch.tensor([count_launches() - l0], dtype=torch.int64, device=device)
         dist.all_reduce(lt, op=dist.ReduceOp.MAX)
         launches = int(lt.item())                      # per rank (the ingest rank launches nothing when its share is 0)
@@ -653,12 +688,15 @@ def run_gpu(args):
             "probs_checksum": checksum, "realtime_streams_capacity": value / 100.0,
         }
         line.update(extras)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
 
 
 def main():
+    sys.dont_write_bytecode = True     # the project's modules are imported below this point: no __pycache__ in the (maybe read-only) tree
     # libraries print to stdout on their own (NCCL's version banner, for one): keep the real stdout for the ONE JSON line and
     # send everything else to stderr
     real_stdout = os.dup(1)
